@@ -15,6 +15,10 @@ a ring whose working set (>= 1.3 GB) is far larger than the 126 MB L2, so no L2 
 
 N>1: one process per GPU (torchrun), independent streams, no collective on the data path
 (SURVEY §8e): "scaling": "weak".  `--impl reference` times the reference CPU path instead.
+
+`--dump-outputs DIR` writes what the last timed step returned (rank 0's frames, see dump_outputs) so
+that two builds run with the same arguments can be compared output for output: the input frames
+are generated from fixed seeds.
 """
 import argparse
 import json
@@ -167,6 +171,24 @@ def cpu_baseline(seconds=10.0, threads=None):
             "sample": f"{n} frames of the same workload in {dt:.1f} s, {impl}"}
 
 
+DUMP_SAMPLE = 4 << 20      # sampled bytes of a step's whole output
+
+
+def dump_outputs(path, frames):
+    """frames: the FRAMES_PER_STEP BGRA frames one step wrote.  Saved as float32 (about 50 MB):
+    bgra_last_frame.npy   the step's last frame, (OH, OW, 4)
+    bgra_sample.npy       the bytes at np.unique(default_rng(0).integers(0, n, DUMP_SAMPLE)) of all n output bytes
+                          of the step, frame after frame"""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    out = torch.stack(frames)
+    np.save(os.path.join(path, "bgra_last_frame.npy"), out[-1].view(OH, OW, 4).cpu().numpy().astype(np.float32))
+    idx = np.unique(np.random.default_rng(0).integers(0, out.numel(), DUMP_SAMPLE))
+    sample = out.view(-1)[torch.from_numpy(idx).to(out.device)]
+    np.save(os.path.join(path, "bgra_sample.npy"), sample.cpu().numpy().astype(np.float32))
+
+
 def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
@@ -309,6 +331,9 @@ def run_ours(args):
         torch.cuda.cudart().cudaProfilerStop()
     ms = e0.elapsed_time(e1)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        o = ((args.steps - 1) % (RING // FRAMES_PER_STEP)) * FRAMES_PER_STEP      # what step(args.steps - 1) wrote
+        dump_outputs(args.dump_outputs, ring_out[o:o + FRAMES_PER_STEP])
 
     # ---- sustained: the same launches back to back for >= 2 s (an issue-bound kernel follows the SM clock, and the
     # clock under a seconds-long load is not the burst clock)
@@ -422,7 +447,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the C1 / C4 / C5 block of the line")
     ap.add_argument("--sustained-seconds", type=float, default=2.5)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's output frames to DIR as .npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         run_reference(args)

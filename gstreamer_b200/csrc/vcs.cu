@@ -93,6 +93,14 @@ int upload_axis (const AxisPlan & a, uint32_t **off, int16_t **coef, int16_t **s
 
 int launch_convert (b200_vcs * h, int n, const VcsBatch & batch, cudaStream_t stream);
 
+// the exact-2:1 kernels load luma and semi-planar chroma as 64-bit words (the plan holds plane offsets and strides to
+// multiples of 8); a batch with any frame off an 8-byte boundary runs the generic kernel, whose YUV input path reads bytes
+bool in_dword_aligned (const VcsBatch & batch, int n)
+{
+  for (int i = 0; i < n; i++) if (((uintptr_t) batch.in[i]) & 7) return false;
+  return true;
+}
+
 // packed RGB -> 4:2:0 with every scaler in front of the matrix (the frame does not grow) and no destination rectangle:
 // vcs_rgb420.cuh.  Leaves rgb420_ok false (the generic chain runs) for what the fast kernels decline.
 int prepare_rgb420 (b200_vcs * h)
@@ -162,6 +170,10 @@ int prepare_rgb420 (b200_vcs * h)
 int launch (b200_vcs * h, int n, const VcsBatch & batch, cudaStream_t stream)
 {
   const VcsPlan & p = h->plan;
+  // every kernel that writes packed RGB stores whole 32-bit pixels: refuse a frame off a 4-byte boundary before
+  // anything (the border fill included) touches it.  The plan builder already holds the plane offset and stride to it.
+  if (p.frame_out.format >= B200_VIDEO_FORMAT_RGBx && p.frame_out.format <= B200_VIDEO_FORMAT_ABGR)
+    for (int i = 0; i < n; i++) if (((uintptr_t) batch.out[i]) & 3) return B200_ERR_INVALID_ARG;
   if (p.has_dest && p.fill_border) {
     // border and rectangle are disjoint byte sets: the fill simply goes first on the same stream
     BorderBatch b;
@@ -195,10 +207,10 @@ int launch_convert (b200_vcs * h, int n, const VcsBatch & batch, cudaStream_t st
     bool aligned = true;                                            // 16-byte cp.async of the luma rows
     for (int i = 0; i < n; i++) aligned = aligned && (((uintptr_t) batch.in[i]) & 15) == 0 && (((uintptr_t) batch.out[i]) & 3) == 0;
     if (aligned) return launch_l2tc (h->dev, h->tc, batch, n, stream);
-    if (p.lanczos2_ok && !p.planar) return launch_lanczos2 (h->dev, h->l2, batch, n, stream);
+    if (p.lanczos2_ok && !p.planar && in_dword_aligned (batch, n)) return launch_lanczos2 (h->dev, h->l2, batch, n, stream);
   }
 #endif
-  if (h->variant == 1 && p.lanczos2_ok && !p.yuv_out) {
+  if (h->variant == 1 && p.lanczos2_ok && !p.yuv_out && in_dword_aligned (batch, n)) {
     if (h->l2v2.ready && h->l2.x4) return launch_lanczos2_v2 (h->dev, h->l2, h->l2v2, batch, n, stream);
     if (!p.planar) return launch_lanczos2 (h->dev, h->l2, batch, n, stream);
   }
@@ -288,9 +300,7 @@ int launch_convert (b200_vcs * h, int n, const VcsBatch & batch, cudaStream_t st
     bool word_aligned = true;
     for (int i = 0; i < n; i++) word_aligned = word_aligned && (((uintptr_t) batch.in[i]) & 3) == 0;
     static const bool slow_chain = getenv ("B200_CROSS_GENERIC") != nullptr;     // A/B knob
-    bool dword_aligned = true;
-    for (int i = 0; i < n; i++) dword_aligned = dword_aligned && (((uintptr_t) batch.in[i]) & 7) == 0;
-    if (!slow_chain && dword_aligned && h->variant == 1 && p.lanczos2_ok && h->l2v2.ready && h->l2.x4) {
+    if (!slow_chain && in_dword_aligned (batch, n) && h->variant == 1 && p.lanczos2_ok && h->l2v2.ready && h->l2.x4) {
       const int s = launch_lanczos2_v2 (h->dev, h->l2, h->l2v2, mid, n, stream);      // exact 2:1, 8 taps: the headline kernel without its matrix
       if (s != B200_OK) return s;
     } else if (!slow_chain && word_aligned && h->variant == 2 && p.light_ok) {
@@ -536,7 +546,6 @@ int b200_vcs_create (const b200_video_info * in, const b200_video_info * out,
 #endif
   }
   const VcsPlan & p = h->plan;
-  if (!p.yuv_out && ((p.out.stride[0] & 3) || (p.out.offset[0] & 3))) { delete h; return B200_ERR_UNSUPPORTED; }
   h->device = device;
   // the kernel this plan will run (also reported for host-only handles: caps negotiation dry-runs, CPU tests)
   h->variant = h->plan.lanczos2_ok ? 1 : (h->plan.light_ok ? 2 : (h->plan.ntap_ok ? 3 : 0));

@@ -767,6 +767,10 @@ int build_vcs_plan (const b200_video_info * in, const b200_video_info * out,
     const b200_vcs_config * cfg, VcsPlan * p)
 {
   if (!in || !out || !cfg || !p) return B200_ERR_INVALID_ARG;
+  // packed RGB is written in 32-bit words: the plane and each of its lines must start on a 4-byte boundary
+  // (b200_vcs_convert_batch holds the frame base to the same)
+  if (out->format >= B200_VIDEO_FORMAT_RGBx && out->format <= B200_VIDEO_FORMAT_ABGR && ((out->stride[0] & 3) || (out->offset[0] & 3)))
+    return B200_ERR_INVALID_ARG;
   if (cfg->dest_width == 0 || cfg->dest_height == 0 ||
       (cfg->dest_x == 0 && cfg->dest_y == 0 && cfg->dest_width == out->width && cfg->dest_height == out->height)) {
     int st = build_inner_plan (in, out, cfg, p, false);

@@ -165,7 +165,18 @@ void b200_vcs_destroy (b200_vcs * h);
  * scratch images between its two launches. */
 int b200_vcs_convert (b200_vcs * h, const void *in_frame, void *out_frame, void *cuda_stream);
 /* n independent frames (same caps) in one launch: what a batching element / multi-stream
- * mux feeds; n <= B200_VCS_MAX_BATCH */
+ * mux feeds; n <= B200_VCS_MAX_BATCH.  Slot i reads in_frames[i] and writes out_frames[i] only.
+ *
+ * Frame placement (b200_vcs_convert and _batch alike):
+ *   - packed RGB outputs are written in 32-bit words: the frame base, info.offset[0] and info.stride[0] must be
+ *     multiples of 4.  b200_vcs_create refuses such an offset or stride, convert such a base, with
+ *     B200_ERR_INVALID_ARG before anything is written.
+ *   - packed RGB inputs: the same rule (refused the same way) wherever the conversion has a YUV output.
+ *   - any other base, offset and stride is accepted and gives the same bytes.  The fast kernels need more
+ *     (the exact-2:1 kernels 8-byte aligned YUV planes, the plane and 4:2:0 packing kernels 4- or 8-byte
+ *     aligned frames); a batch in which any frame falls short runs a kernel that reads and writes bytes.
+ *     Device allocations (cudaMalloc, the torch caching allocator) are 256-byte aligned and always take the
+ *     fast kernels. */
 #define B200_VCS_MAX_BATCH 64
 int b200_vcs_convert_batch (b200_vcs * h, int n, const void *const *in_frames,
     void *const *out_frames, void *cuda_stream);

@@ -1,12 +1,13 @@
 // tests/cudaemu/emu/cuda_runtime.h — TEST INFRASTRUCTURE, NOT PRODUCT CODE.
 //
 // A minimal stand-in for the CUDA runtime and the device execution model so that the SAME kernel sources the product
-// compiles with nvcc (vcs_kernels.cuh, vcs_planes.cuh, vcs_down420.cuh and the glue in vcs.cu) can be compiled with g++
-// and have their indexing and integer arithmetic checked against the oracle on a machine without a GPU.  "Device
-// memory" is host memory; a launch runs the blocks of the grid one after another, each block as real threads with a
-// barrier behind __syncthreads().  Nothing in gstreamer_b200/ loads the library built from this; libb200dsp.so has no
-// CPU fallback.  Kernels that use PTX or warp shuffles (the lanczos2 / light / n-tap fast kernels, the audio and
-// compositor kernels) are not emulated.
+// compiles with nvcc (the vcs_*.cuh kernels, comp.cu, ars.cu and the glue in vcs.cu) can be compiled with g++ and have
+// their indexing and integer arithmetic checked against the oracle on a machine without a GPU.  "Device memory" is host
+// memory; a launch runs the blocks of the grid one after another, each block as real threads with a barrier behind
+// __syncthreads().  Warp shuffles, ballots and mma.sync are emulated lane by lane (b200emu::warp_gather / warp_mma_*);
+// inline PTX is not, so kernels that use it take their plain-C branch under B200_CUDA_EMU.  The one kernel left out
+// is vcs_l2tc_kernel (tcgen05 / tensor memory).  Nothing in gstreamer_b200/ loads the library built from this;
+// libb200dsp.so has no CPU fallback.
 #pragma once
 
 #include <pthread.h>
@@ -31,15 +32,17 @@ struct dim3 {
   unsigned x, y, z;
   dim3 (unsigned a = 1, unsigned b = 1, unsigned c = 1) : x (a), y (b), z (c) {}
 };
-struct uint2 { unsigned x, y; };
-struct uint4 { unsigned x, y, z, w; };
-struct int4 { int x, y, z, w; };
-struct int2 { int x, y; };
-struct float2 { float x, y; };
+// CUDA's own alignments (vector_types.h): a load or store of one of these through a pointer that is not a multiple of
+// its alignment faults on the device, and the UBSan build (build_emu.build ("ubsan")) reports it here
+struct alignas (8) uint2 { unsigned x, y; };
+struct alignas (16) uint4 { unsigned x, y, z, w; };
+struct alignas (16) int4 { int x, y, z, w; };
+struct alignas (8) int2 { int x, y; };
+struct alignas (8) float2 { float x, y; };
 struct alignas (16) float4 { float x, y, z, w; };
-struct double2 { double x, y; };
-struct short2 { short x, y; };
-struct short4 { short x, y, z, w; };
+struct alignas (16) double2 { double x, y; };
+struct alignas (4) short2 { short x, y; };
+struct alignas (8) short4 { short x, y, z, w; };
 
 extern thread_local uint3_emu threadIdx, blockIdx;
 extern thread_local dim3 blockDim, gridDim;

@@ -729,3 +729,76 @@ def test_planar_422_444_to_semi_planar_420(emu, size):
             for site in (1, 2):
                 check(run(emu, fi, fo, size, method, frame, site=site), expected(fi, fo, size, method, frame, site=site),
                       f"{fi}->{fo} m{method} site{site}")
+
+
+# ---- 8. batches: every slot reads its own frame, one handle serves batches of changing sizes -----------------------------
+# (in, out, size, method, kernel variant forced or None, input chroma site, output chroma site, destination rectangle)
+BATCH_ROUTES = {
+    "generic": ("NV12", "BGRA", (40, 30, 24, 18), 3, 0, 2, None, None),
+    "lanczos2-v2": ("NV12", "BGRA", (256, 64, 128, 32), 3, None, 2, None, None),
+    "lanczos2-v2-planar": ("I420", "RGBA", (256, 64, 128, 32), 3, None, 2, None, None),
+    "light": ("NV12", "BGRA", (96, 54, 64, 36), 1, None, 2, None, None),
+    "ntap": ("NV12", "BGRA", (96, 54, 64, 36), 3, None, 2, None, None),
+    "l2mma": ("NV12", "BGRA", (128, 48, 64, 24), 3, 6, 2, None, None),
+    "planes-fast": ("I420", "YV12", (70, 40, 35, 20), 3, None, None, None, None),
+    "chain-lanczos2-v2": ("NV12", "I420", (256, 64, 128, 32), 3, None, 2, None, None),
+    "chain-extra-row": ("NV12", "I420", (40, 29, 24, 29), 1, None, 1, 1, None),
+    "rgb420": ("BGRA", "NV12", (40, 30, 40, 30), 1, None, None, None, None),
+    "rgb420-scaled": ("RGBA", "I420", (48, 36, 24, 18), 3, None, None, None, None),
+    "rgb420-pre1": ("BGRA", "NV12", (24, 18, 40, 30), 1, None, None, None, None),
+    "rgb420-pre2": ("UYVY", "I420", (48, 36, 24, 18), 1, None, None, 1, None),
+    "yuy2-420": ("YUY2", "I420", (40, 30, 40, 30), 1, None, 1, None, None),
+    "borders-rgb": ("NV12", "BGRA", (40, 30, 40, 40), 1, None, 1, None, (0, 5, 40, 30)),
+    "borders-420": ("NV12", "I420", (40, 30, 40, 40), 1, None, 1, 1, (0, 4, 40, 30)),
+}
+
+
+@pytest.mark.parametrize("route", list(BATCH_ROUTES))
+def test_batches_of_distinct_frames(emu, route, monkeypatch):
+    """n = 3 distinct frames in one b200_vcs_convert_batch, then n = 2, 5, 1, 5 on the same handle (the chain's and the
+    rgb420 pre-pass's scratch images grow, stay, shrink and grow back); every slot against the oracle of its own frame,
+    outputs 256 bytes apart with the gaps checked"""
+    from gstreamer_b200 import _lib
+    fi, fo, size, method, force, site, out_site, dest = BATCH_ROUTES[route]
+    iw, ih, W, H = size
+    ii, oi = _lib.VideoInfoC(), _lib.VideoInfoC()
+    assert emu.b200_video_info_set_format(C.byref(ii), ob.FMT[fi], iw, ih) == 0
+    assert emu.b200_video_info_set_format(C.byref(oi), ob.FMT[fo], W, H) == 0
+    if site is not None:
+        ii.chroma_site = site
+    if fi in YUV and fo in YUV:
+        oi.color_matrix, oi.color_range, oi.chroma_site = ii.color_matrix, ii.color_range, ii.chroma_site
+    if fi in YUV_422_444 and fo in YUV:
+        oi.color_matrix, oi.color_range = ii.color_matrix, ii.color_range
+    if out_site is not None:
+        oi.chroma_site = out_site
+    cfg = _lib.VcsConfigC()
+    emu.b200_vcs_config_init(C.byref(cfg))
+    cfg.method = method
+    if dest:
+        cfg.dest_x, cfg.dest_y, cfg.dest_width, cfg.dest_height = dest
+    h = C.c_void_p()
+    assert emu.b200_vcs_create(C.byref(ii), C.byref(oi), C.byref(cfg), 0, C.byref(h)) == 0
+    try:
+        if force is not None:
+            assert emu.b200_vcs_set_kernel_variant(h, force) == 0
+        osz = emu.b200_video_info_size(C.byref(oi))
+        pitch = (osz + 256 + 255) & ~255
+        seed = 0
+        for n in (3, 2, 5, 1, 5):
+            frames = [frame_for(fi, iw, ih, 200 + seed + k) for k in range(n)]
+            seed += n
+            buf = np.full(pitch * n + 256, 0x5A, dtype=np.uint8)
+            base = (-buf.ctypes.data) % 256
+            ins = (C.c_void_p * n)(*[f.ctypes.data for f in frames])
+            outs = (C.c_void_p * n)(*[buf.ctypes.data + base + k * pitch for k in range(n)])
+            assert emu.b200_vcs_convert_batch(h, n, ins, outs, None) == 0
+            for k, f in enumerate(frames):
+                got = buf[base + k * pitch: base + k * pitch + osz]
+                want = expected(fi, fo, size, method, f, dest=dest, border=0xff000000, site=site, out_site=out_site) if dest else \
+                    expected(fi, fo, size, method, f, site=site, out_site=out_site,
+                             colorimetry=(oi.color_matrix, oi.color_range, oi.chroma_site) if fi in RGB and fo in YUV else None)
+                check(got, want, f"{route} n={n} slot {k}")
+                assert (buf[base + k * pitch + osz: base + (k + 1) * pitch] == 0x5A).all(), f"{route} n={n}: slot {k} wrote past its frame"
+    finally:
+        emu.b200_vcs_destroy(h)

@@ -82,17 +82,28 @@ def test_cross_family_matches_oracle(cuda_device, pair, size, method):
 
 
 def test_cross_family_batch(cuda_device):
+    """distinct frames in batches of 5, 2 and 5 on ONE handle: the second batch reuses the scratch images of the first,
+    the third grows them back"""
+    import torch
+    import gstreamer_b200 as g
     size = (640, 360, 426, 240)
     pair = ("NV12", "I420")
-    frame = random_frame(pair, 640, 360, 9)
-    want = expected(size, 3, frame, pair, 2, 2)
-    outs, oi = convert(size, 3, frame, pair, 2, 2, batch=5)
-    for o in outs:
-        assert not planes_equal(o, want, oi, 426, 240, False)
-    # a second, smaller batch on the same handle reuses the scratch images
-    outs, oi = convert(size, 3, frame, pair, 2, 2, batch=2)
-    for o in outs:
-        assert not planes_equal(o, want, oi, 426, 240, False)
+    el = g.CudaVideoConvertScale(add_borders=False, method=3, cuda_device_id=0)
+    ii, oi = g.VideoInfo(ob.FMT[pair[0]], 640, 360), g.VideoInfo(ob.FMT[pair[1]], 426, 240)
+    ii.set_colorimetry(chroma_site=2)
+    oi.set_colorimetry(matrix=ii.c.color_matrix, chroma_site=2)
+    el.set_info(ii, oi)
+    assert int(el.plan_info().kernel_variant) == 5
+    seed = 9
+    for batch in (5, 2, 5):
+        frames = [random_frame(pair, 640, 360, seed + k) for k in range(batch)]
+        seed += batch
+        dst = [torch.full((oi.size,), 0x5A, dtype=torch.uint8, device="cuda") for _ in frames]
+        el.transform_frames([torch.from_numpy(f).cuda() for f in frames], dst)
+        torch.cuda.synchronize()
+        for k, (f, d) in enumerate(zip(frames, dst)):
+            bad = planes_equal(d.cpu().numpy(), expected(size, 3, f, pair, 2, 2), oi, 426, 240, False)
+            assert not bad, f"batch of {batch}, slot {k}: {bad}"
 
 
 def test_cross_family_refusals(cuda_device):
